@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- measures the colour-conversion hot path on B200 (see DESIGN.md "Measurement").
 
-    python bench.py --gpus N --steps K --warmup W [--workload c2|c3|c4|c5] [--impl b200|reference]
+    python bench.py --gpus N --steps K --warmup W [--workload c2|c3|c4|c5] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one synthetic frame (or batch) of the workload.  Default workload c2 is
 the configuration BASELINE.json quotes its metric on: 7680x4320 RGB32f -> 12-bit Rec.2100 PQ YCbCr 4:2:0.
@@ -16,6 +16,8 @@ the configuration BASELINE.json quotes its metric on: 7680x4320 RGB32f -> 12-bit
              the libheif stage) on this box's host cores, on a bounded sample -- reported, not a target.
 
 With --impl reference only the CPU arm runs (rank 0 under torchrun; other ranks exit 0).
+--dump-outputs DIR writes what the last timed step computed to DIR/<name>.npy (see dump_outputs): the inputs are seeded,
+so two builds run with the same arguments can be compared output for output.
 Multi-GPU (torchrun, one rank per GPU): frames / tiles are independent, so ranks share nothing on the data path
 ("scaling": "weak": every rank converts its own frame; --mode tile splits ONE frame into row blocks and gathers
 the planes over NCCL, reported separately in `gather`).
@@ -403,6 +405,25 @@ class DeviceRun:
         return events[0].elapsed_time(events[-1]), [events[i].elapsed_time(events[i + 1]) for i in range(steps)]
 
 
+DUMP_ELEMENTS = 15_000_000  # float32 values in all: a dump stays under 64 MB
+
+
+def dump_outputs(directory, torch, wl, outputs):
+    """Writes the arrays a caller of the timed call receives -- decode: "rgb", the RGB32f rows; encode: the "y", "cb", "cr"
+    and "alpha" planes that exist, their codes as float32 -- to directory/<name>.npy.  An array larger than its even share
+    of DUMP_ELEMENTS keeps a fixed, seeded choice of whole rows (in ascending order), the same on every run."""
+    names = ["rgb"] if wl.direction == "decode" else ["y", "cb", "cr", "alpha"]
+    arrays = [(name, t) for name, t in zip(names, outputs) if t is not None]
+    share = DUMP_ELEMENTS // len(arrays)
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays:
+        keep = min(t.shape[0], max(1, share // t.shape[1]))
+        if keep < t.shape[0]:
+            rows = np.sort(np.random.default_rng(0).choice(t.shape[0], keep, replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        np.save(os.path.join(directory, name + ".npy"), t.float().cpu().numpy())
+
+
 def roofline_block(wl, per_launch_ms, traffic=None):
     peak, peak_source = measured_peak()
     mean_ms = statistics.mean(per_launch_ms)
@@ -553,6 +574,8 @@ def run_b200(args, workload, rank, world, local_rank):
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
     elapsed_ms = max_over_ranks([elapsed_ms])[0]
     value = world * wl.pixels * args.steps / (elapsed_ms * 1e-3) / 1e9
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, wl, run.outputs[(args.steps - 1) % run.copies])
 
     # -- e2e: the host-pointer C-ABI call, pinned host buffers, copies inside the timed region
     e2e_steps = max(1, min(args.steps, 10))
@@ -828,7 +851,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--data", choices=("random", "smooth"), default="random",
                     help="c2 only: 'random' (default, SURVEY 8(d): the worst case for the table look-ups) or 'smooth' (supplementary)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32, rank 0, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -5,12 +5,15 @@ ctypes loaders for the two CPU checkers:
   load_restatement()   oracle/liboracle.so       the plain-C restatement (oracle/avif_oracle.c)
   load_reference()     oracle/_ref/libavifref.so the UNMODIFIED reference translation units compiled in place
                                                  (oracle/Makefile), or None when it has not been built
+  load_recorded_reference()                      the restatement, held call by call to the compiled reference's
+                                                 recorded results (tests/golden/reference_digests.npz)
 
 Both expose the same Python surface (class CpuChecker) so a test can run either against the GPU library.
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may import this module;
 the product package never does.
 """
 import ctypes as C
+import hashlib
 import os
 import subprocess
 import sys
@@ -113,6 +116,11 @@ class CpuChecker:
             self._premultiply_table_u16(max_value, int(unpremultiply), out.ctypes.data)
         return out
 
+    def premultiply_samples(self, values, alphas, max_value, unpremultiply=False):
+        """The 16-bit (un)premultiply of each (value, alpha) pair, one call of the scalar function per pair."""
+        fn = self._unpremultiply_u16 if unpremultiply else self._premultiply_u16
+        return np.array([fn(v, a, max_value) for v, a in zip(np.asarray(values).tolist(), np.asarray(alphas).tolist())], np.uint16)
+
     def yuv_coefficients(self, nclx):
         out = np.zeros(3, np.float32)
         self._check(self._get_yuv_coefficients(C.byref(nclx) if nclx is not None else None, out.ctypes.data))
@@ -210,3 +218,121 @@ def load_reference():
 def best_checker():
     """The compiled reference when available, else the restatement."""
     return load_reference() or load_restatement()
+
+
+# ---- the compiled reference's results, recorded -----------------------------------------------------------------
+#
+# The reference's sources are not part of this repository, so oracle/_ref is only built where they are at hand.  Elsewhere
+# the tests that compare with the reference use RecordedReference: the restatement, held call by call to the results the
+# compiled reference returned for the same calls.  tests/golden/reference_digests.npz keeps those results as SHA-256
+# digests (16 bytes of the digest of the call, 16 of the digest of its result), which keeps the comparison bit-exact
+# over inputs far too large to store.  To record them, where oracle/_ref is built:
+#
+#   AVIFGPU_RECORD_REFERENCE=tests/golden/reference_digests.npz \
+#       python -m pytest tests/test_oracle_vs_reference.py tests/test_forward_roundtrip.py -m "not gpu"
+
+REFERENCE_DIGESTS = os.path.join(_ROOT, "tests", "golden", "reference_digests.npz")
+_UNKEYED = ("threads", "pad")  # how the work is split and laid out in memory; the tests hold that neither changes a result
+
+
+def _feed(h, value):
+    """Hashes a value by content: arrays by dtype, shape and bytes, ctypes structures by their bytes."""
+    if isinstance(value, (np.ndarray, np.generic)):
+        value = np.asarray(value)
+        h.update(f"array {value.dtype.str} {value.shape};".encode())
+        h.update(np.ascontiguousarray(value).tobytes())
+    elif isinstance(value, (list, tuple)):
+        h.update(f"list {len(value)};".encode())
+        for item in value:
+            _feed(h, item)
+    elif isinstance(value, C.Structure):
+        h.update(f"{type(value).__name__};".encode() + bytes(value))
+    elif isinstance(value, OracleError):
+        h.update(f"error {value.status} {value};".encode())
+    elif value is None or isinstance(value, (bool, int, float, str, bytes)):
+        h.update(f"{type(value).__name__} {value!r};".encode())
+    else:
+        raise TypeError(f"no digest for {type(value).__name__}")
+
+
+def _digest(*values):
+    h = hashlib.sha256()
+    for value in values:
+        _feed(h, value)
+    return h.digest()[:16]
+
+
+def _call(checker, name, args, kwargs):
+    """(call digest, result digest, result, error) of checker.<name>(*args, **kwargs); an OracleError is a result too."""
+    keyed = sorted((k, v) for k, v in kwargs.items() if k not in _UNKEYED)
+    key = _digest(name, list(args), [list(kv) for kv in keyed])
+    try:
+        result, error = getattr(checker, name)(*args, **kwargs), None
+    except OracleError as raised:
+        result, error = None, raised
+    return key, _digest(error if error is not None else result), result, error
+
+
+class ReferenceRecorder:
+    """Wraps the compiled reference and records the digest of every call and of its result."""
+
+    def __init__(self, reference):
+        self._reference = reference
+        self.digests = {}
+
+    def __getattr__(self, name):
+        if not callable(getattr(self._reference, name)):
+            return getattr(self._reference, name)
+
+        def call(*args, **kwargs):
+            key, outcome, result, error = _call(self._reference, name, args, kwargs)
+            if self.digests.setdefault(key, outcome) != outcome:
+                raise AssertionError(f"{name}: the compiled reference returned two results for one call (threads or pad changed it)")
+            if error is not None:
+                raise error
+            return result
+        return call
+
+    def save(self, path):
+        keys = sorted(self.digests)
+        np.savez_compressed(path, calls=np.frombuffer(b"".join(keys), np.uint8).reshape(-1, 16),
+                            results=np.frombuffer(b"".join(self.digests[k] for k in keys), np.uint8).reshape(-1, 16),
+                            libm=np.array(self._reference.libm_version()))
+
+
+class RecordedReference:
+    """The restatement in the reference's place: each call runs the restatement and fails unless its result is the one the
+    compiled reference recorded for the same call.  A call the recording does not hold fails as well."""
+
+    def __init__(self, port, calls, results):
+        self._port = port
+        self._results = dict(zip(calls, results))
+
+    def __getattr__(self, name):
+        if not callable(getattr(self._port, name)):
+            return getattr(self._port, name)
+
+        def call(*args, **kwargs):
+            key, outcome, result, error = _call(self._port, name, args, kwargs)
+            expected = self._results.get(key)
+            if expected is None:
+                raise AssertionError(f"{name}: no recorded reference result for this call (record again, see oracle.py)")
+            if expected != outcome:
+                raise AssertionError(f"{name}: the restatement's result differs from the compiled reference's recorded one"
+                                     + (f" (the restatement raised: {error})" if error is not None else ""))
+            if error is not None:
+                raise error
+            return result
+        return call
+
+
+def load_recorded_reference():
+    """RecordedReference over tests/golden/reference_digests.npz, or None where this libm is not the one the results were
+    recorded with (float results are only defined together with their libm)."""
+    if "recorded" not in _cache:
+        port = load_restatement()
+        data = np.load(REFERENCE_DIGESTS)
+        same_libm = str(data["libm"]) == port.libm_version()
+        _cache["recorded"] = RecordedReference(port, [bytes(k) for k in data["calls"]], [bytes(r) for r in data["results"]]) \
+            if same_libm else None
+    return _cache["recorded"]

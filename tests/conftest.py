@@ -26,11 +26,24 @@ def port():
 
 @pytest.fixture(scope="session")
 def ref():
+    """The compiled reference (oracle/_ref) where it is built; elsewhere the restatement held to the reference's recorded
+    results (oracle.RecordedReference).  AVIFGPU_RECORD_REFERENCE=<file> records those results from the compiled reference."""
     import oracle
-    checker = oracle.load_reference()
-    if checker is None:
-        pytest.skip("oracle/_ref/libavifref.so not built (reference tree absent)")
-    return checker
+    compiled = oracle.load_reference()
+    record_to = os.environ.get("AVIFGPU_RECORD_REFERENCE")
+    if compiled is None:
+        if record_to:
+            pytest.fail("AVIFGPU_RECORD_REFERENCE needs the compiled reference (oracle/_ref/libavifref.so)")
+        recorded = oracle.load_recorded_reference()
+        if recorded is None:
+            pytest.skip("the reference's results were recorded with another libm and oracle/_ref is not built")
+        yield recorded
+    elif record_to:
+        recorder = oracle.ReferenceRecorder(compiled)
+        yield recorder
+        recorder.save(record_to)
+    else:
+        yield compiled
 
 
 @pytest.fixture(scope="session")

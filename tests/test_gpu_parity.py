@@ -18,21 +18,22 @@ DECODE_CASES = list(cases.decode_cases(cases.SIZES, full=True))
 
 
 def pick(checker_ref, checker_port, reference_ok):
-    """The compiled reference for every case the reference has a path for; the restatement only where it does not.
-    A missing oracle/_ref is an error here, not a quiet downgrade: "bit-identical to the compiled reference" must not
-    turn green against the restatement alone (AVIFGPU_ALLOW_RESTATEMENT=1 opts out explicitly)."""
+    """The compiled reference (or, where oracle/_ref is not built, the restatement held to the reference's recorded
+    results) for every case the reference has a path for; the restatement alone only where it has none.  Having neither
+    is an error here, not a quiet downgrade: "bit-identical to the compiled reference" must not turn green against the
+    restatement alone (AVIFGPU_ALLOW_RESTATEMENT=1 opts out explicitly)."""
     if reference_ok and checker_ref is None:
         if os.environ.get("AVIFGPU_ALLOW_RESTATEMENT") == "1":
             return checker_port
-        pytest.fail("oracle/_ref/libavifref.so is not loaded: build it where the reference tree is mounted (make -C oracle) -- "
-                    "it ships to the GPU box with the snapshot -- or set AVIFGPU_ALLOW_RESTATEMENT=1 to compare against the restatement")
+        pytest.fail("neither oracle/_ref/libavifref.so nor reference results recorded with this libm: build oracle/_ref where the "
+                    "reference's sources are at hand (make -C oracle), or set AVIFGPU_ALLOW_RESTATEMENT=1 to compare against the restatement")
     return checker_ref if reference_ok else checker_port
 
 
 @pytest.fixture(scope="module")
 def checkers():
     import oracle
-    return oracle.load_reference(), oracle.load_restatement()
+    return oracle.load_reference() or oracle.load_recorded_reference(), oracle.load_restatement()
 
 
 @pytest.mark.parametrize("case", ENCODE_CASES, ids=[c[0] for c in ENCODE_CASES])
