@@ -24,20 +24,6 @@
 
 namespace avifgpu
 {
-int LaunchEncodeGeneric(const EncodeParams& params, int hostDepth, void* stream);
-int LaunchDecodeGeneric(const DecodeParams& params, void* stream);
-int LaunchEncodeFast(const EncodeParams& params, int hostDepth, void* stream);   // 0 = not applicable
-int LaunchEncodeFastInteger(const EncodeParams& params, int hostDepth, void* stream); // 0 = not applicable
-int LaunchEncodeFastGray32(const EncodeParams& params, int hostDepth, void* stream);  // 0 = not applicable
-cudaError_t BuildGray16Lut(uint16_t* deviceLut, int smpte428, uint32_t maxCode, void* stream);
-long long VerifyHlgDivisions(void* stream);
-long long VerifyPqRatio(void* stream);
-long long VerifyFastPremultiply(uint32_t maxCode, void* stream);
-long long VerifyGreenDivision(const DecodeParams& params, void* stream);
-int LaunchDecodeFast(const DecodeParams& params, void* stream);                  // 0 = not applicable
-int LaunchDecodeFastInteger(const DecodeParams& params, void* stream);           // 0 = not applicable
-int LaunchDecodeFastTable(const DecodeParams& params, void* stream);             // 0 = not applicable
-int LaunchHlgOotf(int inverse, const float luma[3], float displayGamma, float peak, const float* in, float* out, size_t pixels, void* stream);
 
 namespace
 {

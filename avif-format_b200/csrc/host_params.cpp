@@ -3,7 +3,9 @@
 // reference's do.
 #include "host_params.h"
 
+#include <cassert>
 #include <cstring>
+#include <type_traits>
 
 namespace avifgpu
 {
@@ -333,6 +335,63 @@ int DecodeHostChannels(const avifgpu_decode_desc& d)
 }
 
 int DecodeHostColBytes(const avifgpu_decode_desc& d) { return DecodeHostChannels(d) * ((d.host_depth + 7) / 8); }
+
+// Sample (column, row) of a buffer whose rows are `stride` bytes apart and whose samples are `bytes` wide.
+template <typename Void>
+static Void* SampleAt(Void* base, int64_t stride, int column, int row, int bytes)
+{
+    using Byte = typename std::conditional<std::is_const<Void>::value, const uint8_t, uint8_t>::type;
+    return static_cast<Byte*>(base) + static_cast<int64_t>(row) * stride + static_cast<int64_t>(column) * bytes;
+}
+
+EncodeParams EncodeSubRect(const EncodeParams& p, int hostDepth, int x, int y, int width, int rows)
+{
+    assert((x & p.xs) == 0 && (y & p.ys) == 0);
+    const int sample = p.imageDepth > 8 ? 2 : 1;
+    const bool gray = p.channels <= 2;
+    EncodeParams s = p;
+    s.rows = SampleAt(p.rows, p.rowStride, x, y, p.channels * (hostDepth / 8));
+    // Planar: Y, Cb, Cr, A.  Reference layout: [0] holds all channels of a colour pixel or gray's Y; [3] gray's alpha.
+    s.plane[0] = SampleAt(p.plane[0], p.planeStride[0], x, y, (p.planar || gray ? 1 : p.channels) * sample);
+    if (p.planar)
+    {
+        s.plane[1] = SampleAt(p.plane[1], p.planeStride[1], x >> p.xs, y >> p.ys, sample);
+        s.plane[2] = SampleAt(p.plane[2], p.planeStride[2], x >> p.xs, y >> p.ys, sample);
+    }
+    if (p.hasAlpha && (p.planar || gray))
+    {
+        s.plane[3] = SampleAt(p.plane[3], p.planeStride[3], x, y, sample);
+    }
+    s.width = width;
+    s.rowCount = rows;
+    return s;
+}
+
+DecodeParams DecodeSubRect(const DecodeParams& p, int x, int y, int width, int rows)
+{
+    assert((x & p.xs) == 0);
+    const int sample = p.bitDepth > 8 ? 2 : 1;
+    const bool mono = p.colorspace == AVIFGPU_COLORSPACE_MONOCHROME;
+    const int hostChannels = (mono ? 1 : 3) + (p.hasAlpha ? 1 : 0);
+    DecodeParams s = p;
+    s.rows = SampleAt(p.rows, p.rowStride, x, y, hostChannels * (p.hostDepth / 8));
+    s.plane[0] = SampleAt(p.plane[0], p.planeStride[0], x, y, sample);
+    if (!mono)
+    {
+        // YCbCr chroma, or planar G and B (xs = ys = yPhase = 0)
+        const int chromaRow = (p.yPhase + y) >> p.ys;
+        s.plane[1] = SampleAt(p.plane[1], p.planeStride[1], x >> p.xs, chromaRow, sample);
+        s.plane[2] = SampleAt(p.plane[2], p.planeStride[2], x >> p.xs, chromaRow, sample);
+    }
+    if (p.hasAlpha)
+    {
+        s.plane[3] = SampleAt(p.plane[3], p.planeStride[3], x, y, sample);
+    }
+    s.width = width;
+    s.rowCount = rows;
+    s.yPhase = (p.yPhase + y) & p.ys;
+    return s;
+}
 
 void FillEncodeParams(const avifgpu_encode_desc& d, EncodeParams* p)
 {

@@ -45,6 +45,12 @@ int EncodeHostColBytes(const avifgpu_encode_desc& desc);
 int DecodeHostChannels(const avifgpu_decode_desc& desc);
 int DecodeHostColBytes(const avifgpu_decode_desc& desc);
 
+// The block's pixels [x, x + width) x [y, y + rows) as a block of their own: every pointer moved to that origin.
+// Encode needs x even when chroma is sub-sampled horizontally and y even when vertically; decode needs x even likewise
+// and takes any y (the result's yPhase says where its first row sits in its chroma row).
+EncodeParams EncodeSubRect(const EncodeParams& p, int hostDepth, int x, int y, int width, int rows);
+DecodeParams DecodeSubRect(const DecodeParams& p, int x, int y, int width, int rows);
+
 // Fills the kernel parameter blocks (pointers and row counts are set by the caller).
 void FillEncodeParams(const avifgpu_encode_desc& desc, EncodeParams* params);
 bool FillDecodeParams(const avifgpu_decode_desc& desc, int32_t transfer, DecodeParams* params, std::string* error);

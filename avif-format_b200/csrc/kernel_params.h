@@ -41,6 +41,28 @@ inline cudaError_t AllowDynamicShared(Kernel kernel, int bytes, std::atomic<uint
     }
     return e;
 }
+
+// Runs a counting kernel synchronously: `launch(counter)` enqueues it on `stream` with a zeroed device counter.  Returns
+// the count the kernel left there, or -1 on a CUDA error.
+template <typename Launch>
+inline long long RunCountingKernel(cudaStream_t stream, Launch launch)
+{
+    unsigned long long* counter = nullptr;
+    if (cudaMalloc(&counter, sizeof(unsigned long long)) != cudaSuccess)
+    {
+        return -1;
+    }
+    cudaMemsetAsync(counter, 0, sizeof(unsigned long long), stream);
+    launch(counter);
+    unsigned long long count = 0;
+    const bool ok = cudaMemcpyAsync(&count, counter, sizeof(count), cudaMemcpyDeviceToHost, stream) == cudaSuccess &&
+                    cudaStreamSynchronize(stream) == cudaSuccess;
+    cudaFree(counter);
+    return ok ? static_cast<long long>(count) : -1;
+}
+
+// The 65536-entry code table of Gray16 hosts (kernels_fast_int.cu); enqueued on `stream`.
+cudaError_t BuildGray16Lut(uint16_t* deviceLut, int smpte428, uint32_t maxCode, void* stream);
 #endif
 
 struct EncodeParams
@@ -117,11 +139,42 @@ struct DecodeParams
 // of asking CUDA a second time (which would answer cudaSuccess and turn a failed launch into AVIFGPU_OK).
 int ReportLaunchFailure(int cudaErrorCode);
 
-// Launchers implemented in kernels_*.cu.  They only enqueue work on `stream` and return the number of kernels
-// launched (>= 1) or a negative avifgpu_status.
+// True when `p` and every row `stride` bytes after it are `alignment`-byte aligned (the tuned kernels' vector accesses).
+inline bool Aligned(const void* p, int64_t stride, int alignment)
+{
+    return (reinterpret_cast<uintptr_t>(p) % alignment) == 0 && (stride % alignment) == 0;
+}
+
+// The SM count the persistent grids are sized for: the context's device, or a B200's for a block made without one.
+constexpr int kB200SmCount = 148;
+inline int SmCount(int32_t smCount) { return smCount > 0 ? smCount : kB200SmCount; }
+
+// Launchers.  They only enqueue work on `stream` and return the number of kernels launched or a negative
+// avifgpu_status.  LaunchEncode / LaunchDecode (avifgpu_api.cu) try the tuned launchers in turn, each of which returns 0
+// when it does not cover the configuration, and end with the generic kernel (kernels_generic.cu), which covers all.
 int LaunchEncode(const EncodeParams& params, int hostDepth, void* stream);
 int LaunchDecode(const DecodeParams& params, void* stream);
+int LaunchEncodeGeneric(const EncodeParams& params, int hostDepth, void* stream); // 0 for an empty block
+int LaunchDecodeGeneric(const DecodeParams& params, void* stream);                // 0 for an empty block
+// The generic kernel over what a tuned kernel covering [0, coveredWidth) x [0, coveredRows) left: the right strip (all
+// rows), then the bottom strip (the covered columns).  The number of kernels launched, or a negative status.
+int LaunchEncodeRemainder(const EncodeParams& params, int hostDepth, int coveredWidth, int coveredRows, void* stream);
+int LaunchDecodeRemainder(const DecodeParams& params, int coveredWidth, int coveredRows, void* stream);
+int LaunchEncodeFast(const EncodeParams& params, int hostDepth, void* stream);        // kernels_fast.cu
+int LaunchEncodeFastInteger(const EncodeParams& params, int hostDepth, void* stream); // kernels_fast_int.cu
+int LaunchEncodeFastGray32(const EncodeParams& params, int hostDepth, void* stream);  // kernels_fast_gray32.cu
+int LaunchDecodeFast(const DecodeParams& params, void* stream);                       // kernels_fast_decode.cu
+int LaunchDecodeFastInteger(const DecodeParams& params, void* stream);                // kernels_fast_decode_int.cu
+int LaunchDecodeFastTable(const DecodeParams& params, void* stream);                  // kernels_fast_decode_table.cu
 int LaunchTransfer(int function, float param, const float* in, float* out, size_t count, void* stream);
+int LaunchHlgOotf(int inverse, const float luma[3], float displayGamma, float peak, const float* in, float* out, size_t pixels, void* stream);
+
+// One-time exhaustive checks behind the tuned kernels' arithmetic shortcuts.  Synchronous: the number of disagreements
+// (0 = verified) or -1 on a CUDA error.
+long long VerifyHlgDivisions(void* stream);                              // HLGToLinearUnit's fast divisions
+long long VerifyPqRatio(void* stream);                                   // PqRatioPair's division, every x the PQ decode makes
+long long VerifyGreenDivision(const DecodeParams& params, void* stream); // the green division of one matrix, depth, range
+long long VerifyFastPremultiply(uint32_t maxCode, void* stream);         // FastPremultiplyBiased for one bit depth
 
 } // namespace avifgpu
 

@@ -130,14 +130,7 @@ cudaError_t DispatchClip(const FastEncodeParams& fp, int xs, int ys, int smCount
     return LaunchClipKernel<0, 0>(fp, smCount, stream);
 }
 
-bool Aligned(const void* p, int64_t stride, int alignment)
-{
-    return (reinterpret_cast<uintptr_t>(p) % alignment) == 0 && (stride % alignment) == 0;
-}
-
 } // namespace
-
-int LaunchEncodeGeneric(const EncodeParams& params, int hostDepth, void* stream);
 
 // Returns the number of kernels launched, 0 if this configuration is not covered, or a negative status.
 int LaunchEncodeFast(const EncodeParams& p, int hostDepth, void* streamHandle)
@@ -173,23 +166,13 @@ int LaunchEncodeFast(const EncodeParams& p, int hostDepth, void* streamHandle)
             return 0;
         }
         const int curve = p.transfer == AVIFGPU_TRANSFER_PQ ? kCurveLinearToPQ : kCurveLinearToSMPTE428;
-        const cudaError_t e = LaunchFastEncodeFlatInterleaved(fp, curve, p.smCount > 0 ? p.smCount : 148, stream);
+        const cudaError_t e = LaunchFastEncodeFlatInterleaved(fp, curve, SmCount(p.smCount), stream);
         if (e != cudaSuccess)
         {
             return ReportLaunchFailure(static_cast<int>(e));
         }
-        int launched = 1;
-        if (width4 < p.width)
-        {
-            EncodeParams strip = p;
-            strip.rows = static_cast<const uint8_t*>(p.rows) + static_cast<int64_t>(width4) * 12;
-            strip.width = p.width - width4;
-            strip.plane[0] = static_cast<uint8_t*>(p.plane[0]) + static_cast<int64_t>(width4) * 6;
-            const int n = LaunchEncodeGeneric(strip, hostDepth, streamHandle);
-            if (n < 0) return n;
-            launched += n;
-        }
-        return launched;
+        const int n = LaunchEncodeRemainder(p, hostDepth, width4, p.rowCount, streamHandle);
+        return n < 0 ? n : 1 + n;
     }
     if (hostDepth != 32 || !p.planar || (p.channels != 3 && !rgba) || (p.channels == 3 && p.hasAlpha) || p.imageDepth <= 8)
     {
@@ -255,7 +238,7 @@ int LaunchEncodeFast(const EncodeParams& p, int hostDepth, void* streamHandle)
         fp.premultiply = p.premultiply;
     }
 
-    const int smCount = p.smCount > 0 ? p.smCount : 148;
+    const int smCount = SmCount(p.smCount);
     cudaError_t e;
     if (rgba)
     {
@@ -281,38 +264,9 @@ int LaunchEncodeFast(const EncodeParams& p, int hostDepth, void* streamHandle)
     {
         return ReportLaunchFailure(static_cast<int>(e));
     }
-    int launched = 1;
-
-    // Edges the tile kernel does not cover go through the generic kernel as sub-rectangles: the right strip
-    // (width % 4 columns, all rows) and, for vertically sub-sampled chroma, an odd last row.
-    if (width4 < p.width)
-    {
-        EncodeParams strip = p;
-        strip.rows = static_cast<const uint8_t*>(p.rows) + static_cast<int64_t>(width4) * (rgba ? 16 : 12);
-        strip.width = p.width - width4;
-        strip.plane[0] = static_cast<uint8_t*>(p.plane[0]) + static_cast<int64_t>(width4) * 2;
-        strip.plane[1] = static_cast<uint8_t*>(p.plane[1]) + static_cast<int64_t>(width4 >> p.xs) * 2;
-        strip.plane[2] = static_cast<uint8_t*>(p.plane[2]) + static_cast<int64_t>(width4 >> p.xs) * 2;
-        if (rgba) strip.plane[3] = static_cast<uint8_t*>(p.plane[3]) + static_cast<int64_t>(width4) * 2;
-        const int n = LaunchEncodeGeneric(strip, hostDepth, streamHandle);
-        if (n < 0) return n;
-        launched += n;
-    }
-    if (evenRows < p.rowCount)
-    {
-        EncodeParams strip = p;
-        strip.rows = static_cast<const uint8_t*>(p.rows) + static_cast<int64_t>(evenRows) * p.rowStride;
-        strip.rowCount = p.rowCount - evenRows;
-        strip.width = width4;
-        strip.plane[0] = static_cast<uint8_t*>(p.plane[0]) + static_cast<int64_t>(evenRows) * p.planeStride[0];
-        strip.plane[1] = static_cast<uint8_t*>(p.plane[1]) + static_cast<int64_t>(evenRows >> p.ys) * p.planeStride[1];
-        strip.plane[2] = static_cast<uint8_t*>(p.plane[2]) + static_cast<int64_t>(evenRows >> p.ys) * p.planeStride[2];
-        if (rgba) strip.plane[3] = static_cast<uint8_t*>(p.plane[3]) + static_cast<int64_t>(evenRows) * p.planeStride[3];
-        const int n = LaunchEncodeGeneric(strip, hostDepth, streamHandle);
-        if (n < 0) return n;
-        launched += n;
-    }
-    return launched;
+    // The right strip (width % 4 columns) and, for vertically sub-sampled chroma, an odd last row: the generic kernel.
+    const int n = LaunchEncodeRemainder(p, hostDepth, width4, evenRows, streamHandle);
+    return n < 0 ? n : 1 + n;
 }
 
 } // namespace avifgpu

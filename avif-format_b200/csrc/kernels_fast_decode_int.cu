@@ -586,14 +586,7 @@ cudaError_t LaunchStream(const StreamDecodeParams& sp, int smCount, cudaStream_t
     return cudaGetLastError();
 }
 
-bool Aligned(const void* p, int64_t stride, int alignment)
-{
-    return (reinterpret_cast<uintptr_t>(p) % alignment) == 0 && (stride % alignment) == 0;
-}
-
 } // namespace
-
-int LaunchDecodeGeneric(const DecodeParams& params, void* stream);
 
 // Monochrome and planar-RGB images for the integer hosts (no premultiplied alpha, depth <= 12: checked by the caller).
 static int LaunchDecodeStream(const DecodeParams& p, void* streamHandle)
@@ -638,7 +631,7 @@ static int LaunchDecodeStream(const DecodeParams& p, void* streamHandle)
     sp.bitDepth = p.bitDepth;
     sp.maxCode = p.maxCode;
     sp.range = p.range;
-    const int smCount = p.smCount > 0 ? p.smCount : 148;
+    const int smCount = SmCount(p.smCount);
     cudaError_t e;
     if (sampleBytes == 1)
     {
@@ -654,24 +647,8 @@ static int LaunchDecodeStream(const DecodeParams& p, void* streamHandle)
     {
         return ReportLaunchFailure(static_cast<int>(e));
     }
-    int launched = 1;
-    if (width8 < p.width)
-    {
-        DecodeParams strip = p;
-        strip.width = p.width - width8;
-        for (int k = 0; k < 4; ++k)
-        {
-            if (p.plane[k] != nullptr)
-            {
-                strip.plane[k] = static_cast<const uint8_t*>(p.plane[k]) + static_cast<int64_t>(width8) * sampleBytes;
-            }
-        }
-        strip.rows = static_cast<uint8_t*>(p.rows) + static_cast<int64_t>(width8) * channels * sampleBytes;
-        const int n = LaunchDecodeGeneric(strip, streamHandle);
-        if (n < 0) return n;
-        launched += n;
-    }
-    return launched;
+    const int n = LaunchDecodeRemainder(p, width8, p.rowCount, streamHandle);
+    return n < 0 ? n : 1 + n;
 }
 
 // Returns the number of kernels launched, 0 if this configuration is not covered, or a negative status.
@@ -727,7 +704,7 @@ int LaunchDecodeFastInteger(const DecodeParams& p, void* streamHandle)
     fp.matrix = p.matrix;
     fp.verifiedGreenDivision = p.verifiedGreenDivision;
 
-    const int smCount = p.smCount > 0 ? p.smCount : 148;
+    const int smCount = SmCount(p.smCount);
     cudaError_t e;
     if (sampleBytes == 1)
     {
@@ -741,43 +718,9 @@ int LaunchDecodeFastInteger(const DecodeParams& p, void* streamHandle)
     {
         return ReportLaunchFailure(static_cast<int>(e));
     }
-    int launched = 1;
-    // Edges go through the generic kernel as sub-rectangles: the right strip (width % 8 columns) and, for vertically
-    // sub-sampled chroma, an odd last row.
-    if (width8 < p.width)
-    {
-        DecodeParams strip = p;
-        strip.width = p.width - width8;
-        strip.plane[0] = static_cast<const uint8_t*>(p.plane[0]) + static_cast<int64_t>(width8) * sampleBytes;
-        strip.plane[1] = static_cast<const uint8_t*>(p.plane[1]) + static_cast<int64_t>(width8 >> p.xs) * sampleBytes;
-        strip.plane[2] = static_cast<const uint8_t*>(p.plane[2]) + static_cast<int64_t>(width8 >> p.xs) * sampleBytes;
-        if (p.hasAlpha)
-        {
-            strip.plane[3] = static_cast<const uint8_t*>(p.plane[3]) + static_cast<int64_t>(width8) * sampleBytes;
-        }
-        strip.rows = static_cast<uint8_t*>(p.rows) + static_cast<int64_t>(width8) * channels * sampleBytes;
-        const int n = LaunchDecodeGeneric(strip, streamHandle);
-        if (n < 0) return n;
-        launched += n;
-    }
-    if (evenRows < p.rowCount)
-    {
-        DecodeParams strip = p;
-        strip.width = width8;
-        strip.rowCount = p.rowCount - evenRows;
-        strip.plane[0] = static_cast<const uint8_t*>(p.plane[0]) + static_cast<int64_t>(evenRows) * p.planeStride[0];
-        strip.plane[1] = static_cast<const uint8_t*>(p.plane[1]) + static_cast<int64_t>(evenRows >> p.ys) * p.planeStride[1];
-        strip.plane[2] = static_cast<const uint8_t*>(p.plane[2]) + static_cast<int64_t>(evenRows >> p.ys) * p.planeStride[2];
-        if (p.hasAlpha)
-        {
-            strip.plane[3] = static_cast<const uint8_t*>(p.plane[3]) + static_cast<int64_t>(evenRows) * p.planeStride[3];
-        }
-        strip.rows = static_cast<uint8_t*>(p.rows) + static_cast<int64_t>(evenRows) * p.rowStride;
-        const int n = LaunchDecodeGeneric(strip, streamHandle);
-        if (n < 0) return n;
-        launched += n;
-    }
-    return launched;
+    // The right strip (width % 8 columns) and, for vertically sub-sampled chroma, an odd last row: the generic kernel.
+    const int n = LaunchDecodeRemainder(p, width8, evenRows, streamHandle);
+    return n < 0 ? n : 1 + n;
 }
 
 } // namespace avifgpu

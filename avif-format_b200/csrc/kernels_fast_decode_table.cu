@@ -159,14 +159,7 @@ cudaError_t LaunchTable(const TableDecodeParams& tp, int smCount, cudaStream_t s
     return cudaGetLastError();
 }
 
-bool Aligned(const void* p, int64_t stride, int alignment)
-{
-    return (reinterpret_cast<uintptr_t>(p) % alignment) == 0 && (stride % alignment) == 0;
-}
-
 } // namespace
-
-int LaunchDecodeGeneric(const DecodeParams& params, void* stream);
 
 // Returns the number of kernels launched, 0 if this configuration is not covered, or a negative status.
 int LaunchDecodeFastTable(const DecodeParams& p, void* streamHandle)
@@ -186,7 +179,6 @@ int LaunchDecodeFastTable(const DecodeParams& p, void* streamHandle)
         return 0;
     }
     const int colours = mono ? 1 : 3;
-    const int channels = colours + (p.hasAlpha ? 1 : 0);
     for (int c = 0; c < colours; ++c)
     {
         if (!Aligned(p.plane[c], p.planeStride[c], 16))
@@ -225,7 +217,7 @@ int LaunchDecodeFastTable(const DecodeParams& p, void* streamHandle)
     tp.gammaMinusOne = p.gammaMinusOne;
     tp.hlgPeak = p.hlgPeak;
     tp.premultiplied = p.premultiplied;
-    const int smCount = p.smCount > 0 ? p.smCount : 148;
+    const int smCount = SmCount(p.smCount);
     cudaError_t e;
     if (mono) e = p.hasAlpha ? LaunchTable<1, 1>(tp, smCount, stream) : LaunchTable<1, 0>(tp, smCount, stream);
     else e = p.hasAlpha ? LaunchTable<3, 1>(tp, smCount, stream) : LaunchTable<3, 0>(tp, smCount, stream);
@@ -233,24 +225,8 @@ int LaunchDecodeFastTable(const DecodeParams& p, void* streamHandle)
     {
         return ReportLaunchFailure(static_cast<int>(e));
     }
-    int launched = 1;
-    if (width8 < p.width)
-    {
-        DecodeParams strip = p;
-        strip.width = p.width - width8;
-        for (int k = 0; k < 4; ++k)
-        {
-            if (p.plane[k] != nullptr)
-            {
-                strip.plane[k] = static_cast<const uint8_t*>(p.plane[k]) + static_cast<int64_t>(width8) * 2;
-            }
-        }
-        strip.rows = static_cast<uint8_t*>(p.rows) + static_cast<int64_t>(width8) * (4 * channels);
-        const int n = LaunchDecodeGeneric(strip, streamHandle);
-        if (n < 0) return n;
-        launched += n;
-    }
-    return launched;
+    const int n = LaunchDecodeRemainder(p, width8, p.rowCount, streamHandle);
+    return n < 0 ? n : 1 + n;
 }
 
 } // namespace avifgpu

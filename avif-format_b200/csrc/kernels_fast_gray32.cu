@@ -221,11 +221,6 @@ __global__ void __launch_bounds__(PQ ? kGrayTableThreads : kGrayClipThreads) Enc
     }
 }
 
-bool Aligned(const void* p, int64_t stride, int alignment)
-{
-    return (reinterpret_cast<uintptr_t>(p) % alignment) == 0 && (stride % alignment) == 0;
-}
-
 template <int CHANNELS, int PQ>
 cudaError_t LaunchGray32(const Gray32Params& gp, size_t shared, int smCount, cudaStream_t stream)
 {
@@ -248,8 +243,6 @@ cudaError_t LaunchGray32(const Gray32Params& gp, size_t shared, int smCount, cud
 }
 
 } // namespace
-
-int LaunchEncodeGeneric(const EncodeParams& params, int hostDepth, void* stream);
 
 // Returns the number of kernels launched, 0 if this configuration is not covered, or a negative status.
 int LaunchEncodeFastGray32(const EncodeParams& p, int hostDepth, void* streamHandle)
@@ -297,7 +290,7 @@ int LaunchEncodeFastGray32(const EncodeParams& p, int hostDepth, void* streamHan
             return 0;
         }
     }
-    const int smCount = p.smCount > 0 ? p.smCount : 148;
+    const int smCount = SmCount(p.smCount);
     cudaError_t e;
     if (p.channels == 2) e = pq ? LaunchGray32<2, 1>(gp, shared, smCount, stream) : LaunchGray32<2, 0>(gp, shared, smCount, stream);
     else e = pq ? LaunchGray32<1, 1>(gp, shared, smCount, stream) : LaunchGray32<1, 0>(gp, shared, smCount, stream);
@@ -305,19 +298,8 @@ int LaunchEncodeFastGray32(const EncodeParams& p, int hostDepth, void* streamHan
     {
         return ReportLaunchFailure(static_cast<int>(e));
     }
-    int launched = 1;
-    if (width4 < p.width)
-    {
-        EncodeParams strip = p;
-        strip.rows = static_cast<const uint8_t*>(p.rows) + static_cast<int64_t>(width4) * (4 * p.channels);
-        strip.width = p.width - width4;
-        strip.plane[0] = static_cast<uint8_t*>(p.plane[0]) + static_cast<int64_t>(width4) * 2;
-        if (p.channels == 2) strip.plane[3] = static_cast<uint8_t*>(p.plane[3]) + static_cast<int64_t>(width4) * 2;
-        const int n = LaunchEncodeGeneric(strip, hostDepth, streamHandle);
-        if (n < 0) return n;
-        launched += n;
-    }
-    return launched;
+    const int n = LaunchEncodeRemainder(p, hostDepth, width4, p.rowCount, streamHandle);
+    return n < 0 ? n : 1 + n;
 }
 
 } // namespace avifgpu

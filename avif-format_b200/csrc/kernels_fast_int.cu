@@ -658,11 +658,6 @@ cudaError_t LaunchGrayInt(const Rgb16Params& rp, int channels, int smCount, cuda
     return cudaGetLastError();
 }
 
-bool Aligned(const void* p, int64_t stride, int alignment)
-{
-    return (reinterpret_cast<uintptr_t>(p) % alignment) == 0 && (stride % alignment) == 0;
-}
-
 template <typename HostT, typename PlaneT, int CHANNELS, int PREMULTIPLY>
 cudaError_t LaunchRgbInt(const Rgb16Params& rp, int xs, int ys, int smCount, cudaStream_t stream)
 {
@@ -687,25 +682,10 @@ cudaError_t LaunchRgbIntChannels(const Rgb16Params& rp, int channels, bool premu
 
 } // namespace
 
-int LaunchEncodeGeneric(const EncodeParams& params, int hostDepth, void* stream);
-
-// Runs the exhaustive comparison behind FastPremultiplyBiased for one bit depth; returns the number of disagreements
-// (0 = verified) or -1 on a CUDA error.  Synchronous.
 long long VerifyFastPremultiply(uint32_t maxCode, void* streamHandle)
 {
     cudaStream_t stream = static_cast<cudaStream_t>(streamHandle);
-    unsigned long long* counter = nullptr;
-    if (cudaMalloc(&counter, sizeof(unsigned long long)) != cudaSuccess)
-    {
-        return -1;
-    }
-    cudaMemsetAsync(counter, 0, sizeof(unsigned long long), stream);
-    VerifyFastPremultiplyKernel<<<148 * 8, 256, 0, stream>>>(maxCode, counter);
-    unsigned long long bad = 0;
-    const bool ok = cudaMemcpyAsync(&bad, counter, sizeof(bad), cudaMemcpyDeviceToHost, stream) == cudaSuccess &&
-                    cudaStreamSynchronize(stream) == cudaSuccess;
-    cudaFree(counter);
-    return ok ? static_cast<long long>(bad) : -1;
+    return RunCountingKernel(stream, [&](unsigned long long* counter) { VerifyFastPremultiplyKernel<<<148 * 8, 256, 0, stream>>>(maxCode, counter); });
 }
 
 cudaError_t BuildGray16Lut(uint16_t* deviceLut, int smpte428, uint32_t maxCode, void* streamHandle)
@@ -722,7 +702,7 @@ int LaunchEncodeFastInteger(const EncodeParams& p, int hostDepth, void* streamHa
     {
         return 0;
     }
-    const int smCount = p.smCount > 0 ? p.smCount : 148;
+    const int smCount = SmCount(p.smCount);
 
     if (hostDepth == 16 && p.imageDepth > 8 && p.channels == 1 && !p.planar)
     {
@@ -748,19 +728,8 @@ int LaunchEncodeFastInteger(const EncodeParams& p, int hostDepth, void* streamHa
         {
             return ReportLaunchFailure(static_cast<int>(launchError));
         }
-        int launched = 1;
-        const int covered = gp.chunksPerRow * 8;
-        if (covered < p.width)
-        {
-            EncodeParams strip = p;
-            strip.rows = static_cast<const uint8_t*>(p.rows) + static_cast<int64_t>(covered) * 2;
-            strip.width = p.width - covered;
-            strip.plane[0] = static_cast<uint8_t*>(p.plane[0]) + static_cast<int64_t>(covered) * 2;
-            const int n = LaunchEncodeGeneric(strip, hostDepth, streamHandle);
-            if (n < 0) return n;
-            launched += n;
-        }
-        return launched;
+        const int n = LaunchEncodeRemainder(p, hostDepth, gp.chunksPerRow * 8, p.rowCount, streamHandle);
+        return n < 0 ? n : 1 + n;
     }
 
     // Gray(+A) hosts in the reference layout (Y plane [0], alpha plane [3]); premultiplication and the Gray16 SMPTE 428
@@ -803,19 +772,8 @@ int LaunchEncodeFastInteger(const EncodeParams& p, int hostDepth, void* streamHa
         {
             return ReportLaunchFailure(static_cast<int>(e));
         }
-        int launched = 1;
-        if (width8 < p.width)
-        {
-            EncodeParams strip = p;
-            strip.rows = static_cast<const uint8_t*>(p.rows) + static_cast<int64_t>(width8) * p.channels * hostBytes;
-            strip.width = p.width - width8;
-            strip.plane[0] = static_cast<uint8_t*>(p.plane[0]) + static_cast<int64_t>(width8) * planeBytes;
-            if (p.channels == 2) strip.plane[3] = static_cast<uint8_t*>(p.plane[3]) + static_cast<int64_t>(width8) * planeBytes;
-            const int n = LaunchEncodeGeneric(strip, hostDepth, streamHandle);
-            if (n < 0) return n;
-            launched += n;
-        }
-        return launched;
+        const int n = LaunchEncodeRemainder(p, hostDepth, width8, p.rowCount, streamHandle);
+        return n < 0 ? n : 1 + n;
     }
 
     // The biased-truncation trick needs non-negative intermediates: true for every matrix with kr, kg, kb >= 0
@@ -873,36 +831,8 @@ int LaunchEncodeFastInteger(const EncodeParams& p, int hostDepth, void* streamHa
         {
             return ReportLaunchFailure(static_cast<int>(e));
         }
-        int launched = 1;
-        const int colBytes = p.channels * hostBytes;
-        if (width8 < p.width)
-        {
-            EncodeParams strip = p;
-            strip.rows = static_cast<const uint8_t*>(p.rows) + static_cast<int64_t>(width8) * colBytes;
-            strip.width = p.width - width8;
-            strip.plane[0] = static_cast<uint8_t*>(p.plane[0]) + static_cast<int64_t>(width8) * planeBytes;
-            strip.plane[1] = static_cast<uint8_t*>(p.plane[1]) + static_cast<int64_t>(width8 >> p.xs) * planeBytes;
-            strip.plane[2] = static_cast<uint8_t*>(p.plane[2]) + static_cast<int64_t>(width8 >> p.xs) * planeBytes;
-            if (p.channels == 4) strip.plane[3] = static_cast<uint8_t*>(p.plane[3]) + static_cast<int64_t>(width8) * planeBytes;
-            const int n = LaunchEncodeGeneric(strip, hostDepth, streamHandle);
-            if (n < 0) return n;
-            launched += n;
-        }
-        if (evenRows < p.rowCount)
-        {
-            EncodeParams strip = p;
-            strip.rows = static_cast<const uint8_t*>(p.rows) + static_cast<int64_t>(evenRows) * p.rowStride;
-            strip.rowCount = p.rowCount - evenRows;
-            strip.width = width8;
-            strip.plane[0] = static_cast<uint8_t*>(p.plane[0]) + static_cast<int64_t>(evenRows) * p.planeStride[0];
-            strip.plane[1] = static_cast<uint8_t*>(p.plane[1]) + static_cast<int64_t>(evenRows >> p.ys) * p.planeStride[1];
-            strip.plane[2] = static_cast<uint8_t*>(p.plane[2]) + static_cast<int64_t>(evenRows >> p.ys) * p.planeStride[2];
-            if (p.channels == 4) strip.plane[3] = static_cast<uint8_t*>(p.plane[3]) + static_cast<int64_t>(evenRows) * p.planeStride[3];
-            const int n = LaunchEncodeGeneric(strip, hostDepth, streamHandle);
-            if (n < 0) return n;
-            launched += n;
-        }
-        return launched;
+        const int n = LaunchEncodeRemainder(p, hostDepth, width8, evenRows, streamHandle);
+        return n < 0 ? n : 1 + n;
     }
     return 0;
 }

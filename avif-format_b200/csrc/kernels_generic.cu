@@ -5,6 +5,7 @@
 // they cannot disagree on arithmetic.
 #include "kernel_params.h"
 #include "curve_lookup.cuh"
+#include "host_params.h"
 #include "../../include/avifgpu.h"
 
 #include <cuda_runtime.h>
@@ -613,6 +614,28 @@ int LaunchDecodeGeneric(const DecodeParams& p, void* streamHandle)
     }
     const cudaError_t launchError = cudaGetLastError();
     return launchError == cudaSuccess ? 1 : ReportLaunchFailure(static_cast<int>(launchError));
+}
+
+int LaunchEncodeRemainder(const EncodeParams& p, int hostDepth, int coveredWidth, int coveredRows, void* stream)
+{
+    const int right = LaunchEncodeGeneric(EncodeSubRect(p, hostDepth, coveredWidth, 0, p.width - coveredWidth, p.rowCount), hostDepth, stream);
+    if (right < 0)
+    {
+        return right;
+    }
+    const int bottom = LaunchEncodeGeneric(EncodeSubRect(p, hostDepth, 0, coveredRows, coveredWidth, p.rowCount - coveredRows), hostDepth, stream);
+    return bottom < 0 ? bottom : right + bottom;
+}
+
+int LaunchDecodeRemainder(const DecodeParams& p, int coveredWidth, int coveredRows, void* stream)
+{
+    const int right = LaunchDecodeGeneric(DecodeSubRect(p, coveredWidth, 0, p.width - coveredWidth, p.rowCount), stream);
+    if (right < 0)
+    {
+        return right;
+    }
+    const int bottom = LaunchDecodeGeneric(DecodeSubRect(p, 0, coveredRows, coveredWidth, p.rowCount - coveredRows), stream);
+    return bottom < 0 ? bottom : right + bottom;
 }
 
 int LaunchTransfer(int function, float param, const float* in, float* out, size_t count, void* streamHandle)
